@@ -24,10 +24,11 @@ cp "$REF/train.py" "$OUT/py/train.py"
 for f in forward_gpu.py backward_gpu.py backward_cpu.py forward_cpu.py; do cp "$REF/$f" "$OUT/py/$f"; done
 find "$OUT/py" -name __pycache__ -prune -exec rm -rf {} +
 if [ "${1:-}" = "py" ]; then ls "$OUT" "$OUT/py"; exit 0; fi
-TMP=$(mktemp -d /tmp/refgsplatcu.XXXXXX)
+TMP=$(mktemp -d)
+# the copied sources keep the reference tree's read-only modes: make them removable on exit
+trap 'chmod -R u+w "$TMP"; rm -rf "$TMP"' EXIT
 cp -r "$REF/gsplatcu" "$TMP/src"
 cd "$TMP/src"
 TORCH_CUDA_ARCH_LIST="10.0a" MAX_JOBS=4 python setup.py build_ext --build-lib "$OUT" --build-temp "$TMP/build" > "$TMP/build.log" 2>&1 \
   || { tail -30 "$TMP/build.log"; exit 1; }
 ls -la "$OUT"
-rm -rf "$TMP"

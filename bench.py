@@ -4,7 +4,7 @@
 A "step" is one pass of the hot path over one synthetic view: parameters -> image ->
 (given dL/dimage) -> gradients of every Gaussian parameter.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 ours, N == 1   config[1] of BASELINE.json: 1M synthetic Gaussians, 1920x1080, SH degree 3.
                `value`/`e2e` time the fused path (GSFunctionFused: gsb_preprocess_forward,
@@ -32,6 +32,7 @@ import os
 import statistics
 import subprocess
 import sys
+import tempfile
 import threading
 import time
 
@@ -44,7 +45,6 @@ METRIC = "rendered Mpixels/s fwd+bwd @1M Gaussians 1080p; grad max-rel-err vs CP
 N_GAUSS, WIDTH, HEIGHT, SH_DIM = 1_000_000, 1920, 1080, 48
 CROP_ROWS = HEIGHT  # CPU arm: the whole frame (a few seconds per pass with OpenMP on the host cores)
 CROP_Y0 = 0
-CPU_BUDGET_S = 150.0  # the reference arm stops adding timed passes once this much CPU time is spent
 
 
 def peaks():
@@ -59,8 +59,8 @@ def cpu_sample(steps=1, warmup=0):
     """forward + backward of the reference algorithm on the host: per-Gaussian stages with
     Jacobians, tile binning + sort, per-pixel compositing, its backward and the Jacobian chain, on
     the whole 1080p view of the 1M-Gaussian scene, OpenMP threads = os.cpu_count() whatever the
-    launcher exported.  Returns (Mpix/s, sec/step, threads, dict with the scene); `steps` timed
-    passes at most -- fewer once CPU_BUDGET_S is spent (the dict says how many)."""
+    launcher exported.  Returns (Mpix/s, sec/step, threads, dict with the scene) over `steps` timed
+    passes."""
     from oracle import oracle as orc
     from easygaussiansplatting_b200.scene import synthetic_scene, upstream_gradient
     orc.set_num_threads(os.cpu_count() or 1)
@@ -69,10 +69,8 @@ def cpu_sample(steps=1, warmup=0):
     cy = sc["cy"] - CROP_Y0
     dl = upstream_gradient(WIDTH, HEIGHT, 0)[:, CROP_Y0:CROP_Y0 + CROP_ROWS, :].copy() * (3.0 * WIDTH * HEIGHT)
     f32 = lambda a: np.ascontiguousarray(a, dtype=np.float32)
-    times, t_begin = [], time.perf_counter()
+    times = []
     for it in range(warmup + steps):
-        if times and time.perf_counter() - t_begin > CPU_BUDGET_S:
-            break
         t0 = time.perf_counter()
         us, pcs, depths, Ju = orc.project(sc["pws"], sc["Rcw"], sc["tcw"], sc["fx"], sc["fy"], sc["cx"], cy)
         d32 = f32(depths)
@@ -171,6 +169,21 @@ class ClockSampler:
 
 
 # ------------------------------------------------------------------ our arm
+DUMP_ROWS = 65536  # Gaussians sampled for --dump-outputs: all of dL/dsh alone would be 192 MB
+
+
+def dump_outputs(out_dir, image, per_gaussian):
+    """--dump-outputs: the last timed step's outputs as <out_dir>/<name>.npy, float32.  The image
+    whole; every per-Gaussian array on the same fixed, seeded sample of DUMP_ROWS Gaussians (rows
+    in ascending order), so that two builds run with the same arguments compare output for output."""
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    rows = torch.from_numpy(np.sort(np.random.default_rng(0).choice(N_GAUSS, DUMP_ROWS, replace=False)))
+    np.save(os.path.join(out_dir, "image.npy"), image.detach().float().cpu().numpy())
+    for name, a in per_gaussian.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a.detach()[rows.to(a.device)].float().cpu().numpy())
+
+
 def run_ours(args, rank, world):
     import torch
     import torch.distributed as dist
@@ -222,11 +235,11 @@ def run_ours(args, rank, world):
             for p in leaves:
                 p.grad = None
             cam.grad_exchange = exchange if use_exchange else None
-            image, _ = F.apply(params["pws"], params["shs"], alphas, params["scales"], params["rots"], us0, cam)
+            image, mask = F.apply(params["pws"], params["shs"], alphas, params["scales"], params["rots"], us0, cam)
             image.backward(dl)
             if world > 1 and not use_exchange:
                 allreduce_grads([p.grad for p in leaves])
-            return image
+            return image, mask
         return step
 
     step_fused, step_ops = make_step(GSFunctionFused, use_ex), make_step(GSFunction, False)
@@ -241,7 +254,7 @@ def run_ours(args, rank, world):
             image, ctx = mv.render(cam)
             mv.backward(ctx, dl, last=True)
             mv_out[0] = mv.reduce()
-            return image
+            return image, None
     else:
         step_sel = step_fused
 
@@ -315,10 +328,27 @@ def run_ours(args, rank, world):
     for _ in range(args.warmup):
         step_sel(dl_dev)
     torch.cuda.synchronize()
+    last = {"calls": 0}
+
+    def step_timed():
+        # only the last step's outputs are kept: an image held into the next step would change
+        # which blocks the caching allocator hands out, and with it the timing
+        out = step_sel(dl_dev)
+        last["calls"] += 1
+        if last["calls"] == args.steps:
+            last["out"] = out
     launches0 = lib.gsb_profile_launches(-1)
-    ms_dev = timed(lambda: step_sel(dl_dev), args.steps, 0)
+    ms_dev = timed(step_timed, args.steps, 0)
     launches = lib.gsb_profile_launches(-1) - launches0
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:  # before any later leg replaces the gradients
+        # (us0.grad is left out: it is never reset, so it sums every step run so far)
+        image, mask = last["out"]
+        if world > 1:
+            outs = {k: mv_out[0][k] for k in ("dpws", "dshs", "dalphas", "dscales", "drots")}
+        else:
+            outs = dict(zip(("dpws", "dshs", "dalphas", "dscales", "drots"), (p.grad for p in leaves)), mask=mask)
+        dump_outputs(args.dump_outputs, image, outs)
     ms_e2e = timed(step_e2e, args.steps, max(3, args.warmup // 2))
     cam.Rcw, cam.tcw, cam.twc = T(Rcw), T(tcw), T(twc)
     ms_ops = timed(lambda: step_ops(dl_dev), max(3, args.steps // 2), 3)
@@ -597,21 +627,18 @@ def reference_gpu_block(gpu_index):
     ref_dir = os.path.join(ROOT, "baseline", "_ref")
     if not (os.path.isdir(ref_dir) and any(f.startswith("gsplatcu") and f.endswith(".so") for f in os.listdir(ref_dir))):
         return None
-    out = os.path.join(ROOT, "gpurun_out", "bench_ref_gpu")
-    os.makedirs(os.path.dirname(out), exist_ok=True)
     sampler = ClockSampler(gpu_index)
     sampler.start()
     try:
-        r = subprocess.run([sys.executable, os.path.join(ROOT, "benchmarks", "compare_ref_gpu.py"), "--arm", "ref",
-                            "--iters", "10", "--out", out, "--configs", "config2"],
-                           capture_output=True, text=True, timeout=600)
-        clocks = sampler.stop()
-        if r.returncode != 0:
-            return {"error": r.stderr[-300:]}
-        res = json.load(open(out + ".ref.json"))["config2"]
-        for f in os.listdir(os.path.dirname(out)):  # the arm's raw tensors are scratch
-            if f.startswith("bench_ref_gpu.ref.json.") and f.endswith(".npz"):
-                os.remove(os.path.join(os.path.dirname(out), f))
+        with tempfile.TemporaryDirectory() as tmp:  # the arm's JSON and raw tensors are scratch
+            out = os.path.join(tmp, "bench_ref_gpu")
+            r = subprocess.run([sys.executable, os.path.join(ROOT, "benchmarks", "compare_ref_gpu.py"), "--arm",
+                                "ref", "--iters", "10", "--out", out, "--configs", "config2"],
+                               capture_output=True, text=True, timeout=600)
+            clocks = sampler.stop()
+            if r.returncode != 0:
+                return {"error": r.stderr[-300:]}
+            res = json.load(open(out + ".ref.json"))["config2"]
         return {"what": "the reference's own gsplatcu (unmodified, built for sm_100a) on this GPU: GSFunction.apply "
                         "(6 ops, calc_J=True) + image.backward (splatB + torch Jacobian chain), config 2, CUDA "
                         "events, median of 10",
@@ -678,7 +705,14 @@ def main():
     ap.add_argument("--steps", type=int, default=20)
     ap.add_argument("--warmup", type=int, default=5)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the image and a fixed sample of the parameter gradients of the last timed "
+                         "step to DIR/<name>.npy (float32)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs dumps the GPU path (--impl ours)")
     rank = int(os.environ.get("RANK", 0))
     world = int(os.environ.get("WORLD_SIZE", 1))
     # stdout carries exactly one JSON line: native libraries (NCCL's version banner) write to

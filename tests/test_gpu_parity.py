@@ -394,21 +394,42 @@ def test_config2_full_size_properties_and_oracle():
     assert torch.isfinite(image).all() and ftau.min() >= 0 and ftau.max() <= 1
 
 
-def test_reference_backward_gpu_script_unmodified():
-    """The reference's own parity script backward_gpu.py (81-152: 19 `[OK]` checks against
-    backward_cpu.py at abs 1e-4) and forward_gpu.py (47-60), run UNMODIFIED on this gsplatcu.
-    Needs the copies baseline/build_ref_gpu.sh puts under baseline/_ref/py (they travel with the
-    gpurun snapshot; absent on a box that never saw the reference tree -> skipped)."""
-    import sys
-    sys.path.insert(0, os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "benchmarks"))
-    import run_reference_scripts as rrs
-    if not rrs.available():
-        pytest.skip("baseline/_ref/py not installed")
-    res = rrs.run("ours")
-    b = res["backward_gpu"]
-    assert b["ng"] == 0 and b["ok"] == 19, b["lines"]
-    f = res["forward_gpu"]
-    assert f["image_shape"] == [3, 546, 979] and f["image_max"] > 0.1
+def test_reference_backward_gpu_script_checks():
+    """The 19 checks of the reference's parity script backward_gpu.py (81-152): its operator call
+    sequence on its 4-Gaussian example scene at 32x16, every output and Jacobian, the image and
+    splatB's four gradients against what its backward_cpu.py computed (tests/golden/scripts.npz,
+    make_golden_scripts.py), each with the script's abs-1e-4 `check`.  Then the inference call
+    sequence of forward_gpu.py (47-60) on the same Gaussians at 979x546."""
+    d = dict(np.load(os.path.join(G, "scripts.npz")))
+    g = gsc()
+    fx, fy, cx, cy, W, H = d["cam"]
+    W, H = int(W), int(H)
+    pws, rots, scales, alphas, shs = (t(d[k]) for k in ("pws", "rots", "scales", "alphas", "shs"))
+    Rcw, tcw, twc = t(d["Rcw"]), t(d["tcw"]), t(d["twc"])
+    us, pcs, _, du_dpcs = g.project(pws, Rcw, tcw, fx, fy, cx, cy, True)
+    depths = t(np.array([1, 2, 3, 4]))  # the script's fixed depths, not the projected ones
+    c3, J3r, J3s = g.computeCov3D(rots, scales, depths, True)
+    c2, J2c, J2p = g.computeCov2D(c3, pcs, Rcw, depths, fx, fy, W, H, True)
+    col, Jcs, Jcp = g.sh2Color(shs, pws, twc, True)
+    ci, areas, Jci = g.inverseCov2D(c2, depths, True)
+    image, contrib, ftau, ranges, gsid = g.splat(H, W, us, ci, alphas, depths, col, areas)
+    grads = g.splatB(H, W, us, ci, alphas, depths, col, contrib, ftau, ranges, gsid, t(d["dloss_dgammas"]))
+    got = dict(us=us, pcs=pcs, du_dpcs=du_dpcs, cov3ds=c3, dcov3d_drots=J3r, dcov3d_dscales=J3s, cov2ds=c2,
+               dcov2d_dcov3ds=J2c, dcov2d_dpcs=J2p, colors=col, dcolor_dshs=Jcs, dcolor_dpws=Jcp, cinv2ds=ci,
+               dcinv2d_dcov2ds=Jci, image=image.permute(1, 2, 0))
+    got.update(zip(("dloss_dus", "dloss_dcinv2ds", "dloss_dalphas", "dloss_dcolors"), grads))
+    failed = [k for k, v in got.items() if not np.all(np.abs(n(v).astype(np.float64).reshape(d[k].shape) - d[k]) < 1e-4)]
+    assert len(got) == 19 and not failed, failed
+    # forward_gpu.py: deg-0 colours, its own camera; it passes (height, width) to computeCov2D in that order
+    fx, fy, W, H = 581.6273640151177, 578.140202494143, 979, 546
+    twc = torch.linalg.inv(Rcw) @ (-tcw)
+    us, pcs, depths = g.project(pws, Rcw, tcw, fx, fy, W / 2, H / 2, False)
+    c3 = g.computeCov3D(rots, scales, depths, False)[0]
+    c2 = g.computeCov2D(c3, pcs, Rcw, depths, fx, fy, H, W, False)[0]
+    col = g.sh2Color(shs[:, :3].contiguous(), pws, twc, False)[0]
+    ci, areas = g.inverseCov2D(c2, depths, False)
+    image = g.splat(H, W, us, ci, alphas, depths, col, areas)[0]
+    assert list(image.shape) == [3, 546, 979] and float(image.max()) > 0.1
 
 
 @pytest.mark.parametrize("N,W,H", [(2_000_000, 1920, 1080), (5_000_000, 3840, 2160)])
