@@ -1,7 +1,7 @@
-"""A/B of the N2 (loss) and N3 (density) kernel variants: per-kernel ms from the library's own
-CUDA-event profile + checksums of the outputs, one JSON line.  Variants are selected through the
-environment (GSB_LOSS_VARIANT, GSB_LOSS_STRIP, GSB_DENSITY_VARIANT, GSB_DENSITY_SCAN_VARIANT), so
-one process = one variant:  python benchmarks/ab_n2n3.py [--once] [--hw 1080x1920] [--n 1000000]"""
+"""N2 (loss) and N3 (density) kernels on seeded inputs: per-kernel ms from the library's own
+CUDA-event profile + SHA-1 prefixes of the outputs, one JSON line.  Two builds (GSB_LIB, see
+ab_variants.py) compute the same thing exactly when their `grad_sha`, `cls_slots_sha` and `out_sha`
+agree:  python benchmarks/ab_n2n3.py [--once] [--hw 1080x1920] [--n 1000000]"""
 import argparse
 import ctypes as C
 import hashlib

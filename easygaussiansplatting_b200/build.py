@@ -18,7 +18,7 @@ VARIANT = os.environ.get("GSB_VARIANT", "")
 OBJ = os.path.join(HERE, "_obj" + ("_" + VARIANT if VARIANT else ""))
 LIB = os.path.join(HERE, "libgsplat_b200%s.so" % ("_" + VARIANT if VARIANT else ""))
 SOURCES = ["api.cu", "pergaussian.cu", "fused.cu", "binning.cu", "raster_bwd.cu",
-           "raster_fwd2.cu", "raster_fwd3.cu", "raster_bwd2.cu", "raster_bwd4.cu", "loss.cu", "smallbmm.cu", "density.cu", "comm.cu"]
+           "raster_fwd3.cu", "raster_bwd4.cu", "loss.cu", "smallbmm.cu", "density.cu", "comm.cu"]
 NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
 FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-std=c++17", "-lineinfo",
          "-Xcompiler", "-fPIC", "-Xptxas", "-v", "--expt-relaxed-constexpr",

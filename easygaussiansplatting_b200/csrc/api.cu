@@ -279,14 +279,9 @@ int gsb_splat_render(int H, int W, int N, int64_t P, uint32_t depth_key_max, con
   if (rc) return rc;
   const Rec *recs = P > 0 ? reinterpret_cast<const Rec *>(static_cast<char *>(ws) + SL.recs) : nullptr;
   if (P > 0 && packed_records != nullptr) recs = static_cast<const Rec *>(packed_records);
-  // with P == 0 the workspace may be a dummy: every tile is empty, any variant just writes zeros
-  int *tile_counter = reinterpret_cast<int *>(static_cast<char *>(ws) + SL.counters);
-  // sparse frame (< 48 patches per tile on average): persistent grid + tile queue
-  const int64_t T = (int64_t)((W + GSB_TILE - 1) / GSB_TILE) * ((H + GSB_TILE - 1) / GSB_TILE);
-  int *const work_counter = tile_counter;
-  if (P >= 48 * T) tile_counter = nullptr;
-  return launch_draw(H, W, patch_range_per_tile, recs, gsid_per_patch, image, contrib, final_tau, tile_counter,
-                     work_counter, st);
+  // with P == 0 every tile is empty: the rasterizer only writes zeros
+  int *work = reinterpret_cast<int *>(static_cast<char *>(ws) + SL.counters);
+  return launch_draw(H, W, patch_range_per_tile, recs, gsid_per_patch, image, contrib, final_tau, work, st);
 }
 
 static int splat_forward_impl(int H, int W, int N, const float *us, const float *cinv2ds, const float *alphas,
@@ -314,24 +309,18 @@ static int splat_forward_impl(int H, int W, int N, const float *us, const float 
   if (wait) status_host[0] = status_host[1] = status_host[2] = 0;
   rc = launch_bin(H, W, N, us, depths, areas, bin_ws, BL, st);
   if (rc) return rc;
+  int *work = reinterpret_cast<int *>(static_cast<char *>(ws) + SL.counters);
   if (N == 0) {  // nothing to bin: every tile is empty
     GSB_CUDA_TRY(cudaMemsetAsync(patch_range_per_tile, 0,
                                  sizeof(int32_t) * 2 * (size_t)((W + GSB_TILE - 1) / GSB_TILE) * ((H + GSB_TILE - 1) / GSB_TILE), st));
-    int *work = reinterpret_cast<int *>(static_cast<char *>(ws) + SL.counters);
-    return launch_draw(H, W, patch_range_per_tile, nullptr, gsid_per_patch, image, contrib, final_tau, work, work, st);
+    return launch_draw(H, W, patch_range_per_tile, nullptr, gsid_per_patch, image, contrib, final_tau, work, st);
   }
   rc = launch_sort_and_pack(H, W, N, P_cap, depth_key_cap, us, cinv2ds, alphas, depths, colors, bin_ws, BL, ws, SL,
                             patch_range_per_tile, gsid_per_patch, packed_records == nullptr, &sr, st);
   if (rc) return rc;
   const Rec *recs = packed_records != nullptr ? static_cast<const Rec *>(packed_records)
                                               : reinterpret_cast<const Rec *>(static_cast<char *>(ws) + SL.recs);
-  // sparse frame -> persistent tile queue; the host does not know P yet, the capacity stands in
-  int *tile_counter = reinterpret_cast<int *>(static_cast<char *>(ws) + SL.counters);
-  const int64_t T = (int64_t)((W + GSB_TILE - 1) / GSB_TILE) * ((H + GSB_TILE - 1) / GSB_TILE);
-  int *const work_counter = tile_counter;
-  if (P_cap >= 60 * T) tile_counter = nullptr;
-  rc = launch_draw(H, W, patch_range_per_tile, recs, gsid_per_patch, image, contrib, final_tau, tile_counter,
-                   work_counter, st);
+  rc = launch_draw(H, W, patch_range_per_tile, recs, gsid_per_patch, image, contrib, final_tau, work, st);
   if (rc) return rc;
   if (!wait) return 0;  // enqueue-only (CUDA graph capture): the caller inspects status_host later
   // the sort and the rasterizer are queued; now look at what the binning found
@@ -395,7 +384,7 @@ int gsb_splat_backward(int H, int W, int N, int64_t P, const float *us, const fl
   Rec *recs = reinterpret_cast<Rec *>(base);
   uintptr_t mbase = (base + (size_t)(P_ws > 0 ? N : 1) * sizeof(Rec) + 255) & ~(uintptr_t)255;
   float *moments = moments_out != nullptr ? moments_out : reinterpret_cast<float *>(mbase);
-  int *tile_counter = reinterpret_cast<int *>((mbase + (size_t)N * 9 * sizeof(float) + 255) & ~(uintptr_t)255);
+  int *work = reinterpret_cast<int *>((mbase + (size_t)N * 9 * sizeof(float) + 255) & ~(uintptr_t)255);
   if (P > 0) {
     GSB_REQUIRE(us && alphas && colors && contrib && final_tau && patch_range_per_tile && gsid_per_patch &&
                     dloss_dgammas,
@@ -409,12 +398,9 @@ int gsb_splat_backward(int H, int W, int N, int64_t P, const float *us, const fl
     }
   }
   // P == 0: nothing was drawn; the zeroed moment rows finalise to all-zero gradients
-  const int64_t T = (int64_t)((W + GSB_TILE - 1) / GSB_TILE) * ((H + GSB_TILE - 1) / GSB_TILE);
-  int *const work_counter = tile_counter;  // the warp-autonomous kernel always pulls from a counter
-  if (P >= 48 * T) tile_counter = nullptr;  // dense frame: one CTA per tile (variants 2 / 3)
   return launch_draw_backward(H, W, N, patch_range_per_tile, P > 0 ? recs : nullptr, gsid_per_patch, contrib, final_tau,
-                              dloss_dgammas, cinv2ds, moments, tile_counter, work_counter, dloss_dus, dloss_dcinv2ds,
-                              dloss_dalphas, dloss_dcolors, moments_out == nullptr, st);
+                              dloss_dgammas, cinv2ds, moments, work, dloss_dus, dloss_dcinv2ds, dloss_dalphas,
+                              dloss_dcolors, moments_out == nullptr, st);
 }
 
 // ---- density control + record conversion (density.cu)

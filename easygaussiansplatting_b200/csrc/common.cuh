@@ -1,5 +1,5 @@
-// Shared device helpers for the sm_100a kernels: constants fixed by the reference,
-// mbarrier / bulk-async-copy (TMA 1-D, SASS UBLKCP) PTX wrappers, fast math.
+// Shared device helpers for the sm_100a kernels: constants fixed by the reference, the packed
+// record, fast math, PTX wrappers.
 #pragma once
 #include <cuda_runtime.h>
 #include <stdint.h>
@@ -14,8 +14,8 @@ constexpr float ALPHA_SKIP = 0.002f;  // kernel.cu:246
 constexpr float TAU_STOP = 0.0001f;   // kernel.cu:256
 constexpr float LOG2E = 1.4426950408889634f;
 
-// Packed per-patch record, 48 B, written by pack_records (binning.cu) in sorted order so a
-// tile's records are one contiguous 16-B aligned span -> one cp.async.bulk per batch.
+// Packed per-Gaussian record, 48 B (build_record below), 16-B aligned: the rasterizers gather it
+// with three 16-byte cp.async.
 //   q0 = (ux, uy, gsid bits, alpha)   mean in pixels, Gaussian id, opacity -- exactly the four
 //                              words the backward's moment phase needs per record (one 16-byte copy)
 //   q1 = (a, b, c, thr)        log2(g) = a dx^2 + b dx dy + c dy^2  (conic pre-scaled by
@@ -134,58 +134,9 @@ __device__ __forceinline__ unsigned long long globaltimer_ns() {
   return t;
 }
 
-// ---- mbarrier + bulk async copy (global -> shared), single-CTA forms
+// ---- shared-memory address of a generic pointer (the operand of ld/st.shared and cp.async)
 __device__ __forceinline__ uint32_t smem_u32(const void *p) {
   return static_cast<uint32_t>(__cvta_generic_to_shared(p));
-}
-__device__ __forceinline__ void mbar_init(uint64_t *bar, uint32_t count) {
-  asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(count));
-}
-__device__ __forceinline__ void fence_mbar_init() {
-  asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-}
-__device__ __forceinline__ void fence_proxy_async() {
-  asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-}
-__device__ __forceinline__ void mbar_expect_tx(uint64_t *bar, uint32_t bytes) {
-  asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)),
-               "r"(bytes)
-               : "memory");
-}
-__device__ __forceinline__ bool mbar_try_wait(uint64_t *bar, uint32_t parity) {
-  uint32_t ok;
-  asm volatile(
-      "{\n"
-      ".reg .pred p;\n"
-      "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n"
-      "selp.u32 %0, 1, 0, p;\n"
-      "}\n"
-      : "=r"(ok)
-      : "r"(smem_u32(bar)), "r"(parity)
-      : "memory");
-  return ok != 0;
-}
-__device__ __forceinline__ void mbar_wait(uint64_t *bar, uint32_t parity) {
-  while (!mbar_try_wait(bar, parity)) {
-  }
-}
-// ---- per-thread 16-byte async copies (gather) tracked by an mbarrier: every thread of the
-// CTA issues its copies and then arrives once; the barrier (initialised with the CTA size)
-// completes the phase when all those copies have landed.
-__device__ __forceinline__ void cp_async16(void *dst_smem, const void *src_gmem) {
-  asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(smem_u32(dst_smem)), "l"(src_gmem) : "memory");
-}
-__device__ __forceinline__ void cp_async_mbar_arrive(uint64_t *bar) {
-  asm volatile("cp.async.mbarrier.arrive.noinc.shared::cta.b64 [%0];" ::"r"(smem_u32(bar)) : "memory");
-}
-// 1-D TMA: bytes must be a multiple of 16, both addresses 16-B aligned.
-__device__ __forceinline__ void bulk_g2s(void *dst_smem, const void *src_gmem, uint32_t bytes,
-                                         uint64_t *bar) {
-  asm volatile(
-      "cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::
-          "r"(smem_u32(dst_smem)),
-      "l"(src_gmem), "r"(bytes), "r"(smem_u32(bar))
-      : "memory");
 }
 
 }  // namespace gsb
@@ -199,36 +150,4 @@ __device__ __forceinline__ void bulk_g2s(void *dst_smem, const void *src_gmem, u
 namespace gsb {
 int set_cuda_error(cudaError_t e, const char *what, const char *file, int line);
 int set_arg_error(const char *msg);
-
-// Stage fill of the rasterizers = a gather: lane `tid` of the 128-thread CTA fetches the 48-byte
-// record of Gaussian g into dst[tid]; `bar` flips when all n_valid records have landed.
-//   GSB_GATHER_BULK = 1: one 48-byte cp.async.bulk (TMA, SASS UBLKCP) per record, completion by
-//                        byte count (mbarrier initialised with 1: thread 0 posts the expected bytes)
-//   GSB_GATHER_BULK = 0: three 16-byte cp.async (LDGSTS) per record, every thread arrives once
-//                        (mbarrier initialised with 128)
-#ifndef GSB_GATHER_BULK
-#define GSB_GATHER_BULK 0
-#endif
-constexpr uint32_t GATHER_ARRIVALS = GSB_GATHER_BULK ? 1 : 128;
-__device__ __forceinline__ void gather_record(Rec *dst, const Rec *__restrict__ recs, int g, bool valid,
-                                              int n_valid, uint64_t *bar, int tid) {
-#if GSB_GATHER_BULK
-  if (tid == 0) mbar_expect_tx(bar, (uint32_t)n_valid * (uint32_t)sizeof(Rec));
-  if (valid) {
-    fence_proxy_async();
-    bulk_g2s(dst + tid, recs + g, (uint32_t)sizeof(Rec), bar);
-  }
-#else
-  (void)n_valid;
-  if (valid) {
-    const char *s = reinterpret_cast<const char *>(recs + g);
-    char *d = reinterpret_cast<char *>(dst + tid);
-    cp_async16(d, s);
-    cp_async16(d + 16, s + 16);
-    cp_async16(d + 32, s + 32);
-  }
-  cp_async_mbar_arrive(bar);
-#endif
-}
-
 }  // namespace gsb

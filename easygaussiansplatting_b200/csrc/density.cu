@@ -17,14 +17,8 @@
 // Transcendentals are the accurate expf / logf / sqrtf / IEEE division (no fast-math here):
 // torch's CUDA kernels use the same libdevice routines, which keeps the clone / split values
 // within an ulp of the reference's.
-#include <stdlib.h>
-
 #include "common.cuh"
 #include "kernels.h"
-
-#ifndef GSB_DENSITY_DEFAULT_VARIANT
-#define GSB_DENSITY_DEFAULT_VARIANT 3
-#endif
 
 namespace gsb {
 
@@ -220,44 +214,44 @@ __device__ __forceinline__ float split_offset(const float *__restrict__ q4, cons
 // blockIdx.y, grid-stride over the job's N*w elements, four independent elements in flight
 // per thread (loads first, then stores).  Survivors move to their compacted row; clones /
 // splits additionally produce a new row at K + slot (clones) or K + C + slot (splits): the
-// recomputed value for a parameter, zero for an Adam moment.  I = int32 whenever every
-// element index fits (N < 23 M), which keeps the divisions by the row width single mul.hi.
-template <int A, int SET, typename I>
-__device__ __forceinline__ void apply_job(I N, const uint8_t *__restrict__ cls, const Slot3 *__restrict__ slots,
-                                          I K, I C, const Sets &S, const float *__restrict__ z) {
+// recomputed value for a parameter, zero for an Adam moment.  64-bit element indices: this
+// kernel is the path for N >= 23 M, where N * 45 overflows 32 bits (k_density_apply_rows below).
+template <int A, int SET>
+__device__ __forceinline__ void apply_job(int64_t N, const uint8_t *__restrict__ cls, const Slot3 *__restrict__ slots,
+                                          int64_t K, int64_t C, const Sets &S, const float *__restrict__ z) {
   constexpr int w = kWidth[A];
   constexpr int U = 4;
   const float *__restrict__ src = SET == 0 ? S.p[A] : (SET == 1 ? S.m[A] : S.v[A]);
   float *__restrict__ dst = SET == 0 ? S.dp[A] : (SET == 1 ? S.dm[A] : S.dv[A]);
   if (src == nullptr) return;
-  const I total = N * w;
-  const I stride = (I)gridDim.x * blockDim.x;
-  for (I e0 = (I)blockIdx.x * blockDim.x + threadIdx.x; e0 < total; e0 += stride * U) {
-    I row[U];
+  const int64_t total = N * w;
+  const int64_t stride = (int64_t)gridDim.x * blockDim.x;
+  for (int64_t e0 = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; e0 < total; e0 += stride * U) {
+    int64_t row[U];
     uint8_t cl[U];
     float val[U];
     Slot3 sl[U];
 #pragma unroll
     for (int u = 0; u < U; u++) {
-      const I e = e0 + (I)u * stride;
+      const int64_t e = e0 + (int64_t)u * stride;
       row[u] = e < total ? e / w : 0;
       cl[u] = e < total ? cls[row[u]] : (uint8_t)CLS_PRUNE;
     }
 #pragma unroll
     for (int u = 0; u < U; u++) {
       if (cl[u] == CLS_PRUNE) continue;
-      val[u] = src[e0 + (I)u * stride];
+      val[u] = src[e0 + (int64_t)u * stride];
       sl[u] = slots[row[u]];
     }
 #pragma unroll
     for (int u = 0; u < U; u++) {
       if (cl[u] == CLS_PRUNE) continue;
-      const I i = row[u];
-      const int c = (int)(e0 + (I)u * stride - i * w);
-      dst[(I)sl[u].k * w + c] = val[u];
+      const int64_t i = row[u];
+      const int c = (int)(e0 + (int64_t)u * stride - i * w);
+      dst[(int64_t)sl[u].k * w + c] = val[u];
       if (cl[u] == CLS_KEEP) continue;
       const bool split = cl[u] == CLS_SPLIT;
-      const I r = (split ? K + C + (I)sl[u].s : K + (I)sl[u].c) * w + c;
+      const int64_t r = (split ? K + C + (int64_t)sl[u].s : K + (int64_t)sl[u].c) * w + c;
       float nv = 0.f;
       if (SET == 0) {
         nv = val[u];
@@ -278,12 +272,11 @@ __device__ __forceinline__ void apply_job(I N, const uint8_t *__restrict__ cls, 
   }
 }
 
-template <typename I>
-__global__ void __launch_bounds__(256) k_density_apply(I N, const uint8_t *__restrict__ cls,
-                                                       const Slot3 *__restrict__ slots, I K, I C, Sets S,
+__global__ void __launch_bounds__(256) k_density_apply(int64_t N, const uint8_t *__restrict__ cls,
+                                                       const Slot3 *__restrict__ slots, int64_t K, int64_t C, Sets S,
                                                        const float *__restrict__ z) {
 #define GSB_JOB(a, s) \
-  case 3 * a + s: apply_job<a, s, I>(N, cls, slots, K, C, S, z); break;
+  case 3 * a + s: apply_job<a, s>(N, cls, slots, K, C, S, z); break;
   switch (blockIdx.y) {
     GSB_JOB(0, 0) GSB_JOB(0, 1) GSB_JOB(0, 2) GSB_JOB(1, 0) GSB_JOB(1, 1) GSB_JOB(1, 2)
     GSB_JOB(2, 0) GSB_JOB(2, 1) GSB_JOB(2, 2) GSB_JOB(3, 0) GSB_JOB(3, 1) GSB_JOB(3, 2)
@@ -292,7 +285,7 @@ __global__ void __launch_bounds__(256) k_density_apply(I N, const uint8_t *__res
 #undef GSB_JOB
 }
 
-// ---- row-group variant (default for N < 23 M): a warp moves 32 consecutive Gaussians of one array.
+// ---- row groups (the path for N < 23 M): a warp moves 32 consecutive Gaussians of one array.
 // The per-Gaussian plan (class, survivor slot, new-row slot) is read once per group into a
 // 32-entry shared-memory table instead of once per element (13 B per 4-byte element in the
 // kernel above).  Loads and stores are 4-byte but fully coalesced: lane l handles elements
@@ -302,6 +295,7 @@ __global__ void __launch_bounds__(256) k_density_apply(I N, const uint8_t *__res
 // four components with stride-16-byte stores: quarter-filled sectors, 0.57 ms against the 0.45 ms
 // of the kernel above.)  Elements of pruned Gaussians are not loaded.
 constexpr int DG_WARPS = 8;
+constexpr int DG_PAIRS = 4;  // row pairs of a [*, 45] array in flight per lane (12 loads)
 
 // the value a clone / split writes at its new row (parameters; Adam moments start at 0)
 template <int A>
@@ -322,9 +316,9 @@ __device__ __forceinline__ float new_row_value(float val, bool split, int64_t i,
   return nv;
 }
 
-template <int A, int SET, int FIXED>  // FIXED: 0 = generic loop, else pairs of wide rows in flight per lane
-__device__ __forceinline__ void rows_job(int row0, int rows_here, const int2 *__restrict__ tab, int K, int C,
-                                         const Sets &S, const float *__restrict__ z, int lane) {
+template <int A, int SET>
+__device__ __forceinline__ void rows_job(int row0, const int2 *__restrict__ tab, int K, int C, const Sets &S,
+                                         const float *__restrict__ z, int lane) {
   constexpr int w = kWidth[A];
   const float *__restrict__ src = SET == 0 ? S.p[A] : (SET == 1 ? S.m[A] : S.v[A]);
   float *__restrict__ dst = SET == 0 ? S.dp[A] : (SET == 1 ? S.dm[A] : S.dv[A]);
@@ -340,9 +334,8 @@ __device__ __forceinline__ void rows_job(int row0, int rows_here, const int2 *__
     if (SET == 0) nv = new_row_value<A>(val, cl == CLS_SPLIT, (int64_t)row0 + r, info.y - K - C, col, S, z);
     dst[(size_t)info.y * w + col] = nv;
   };
-  const int2 pruned = make_int2((int)((unsigned)CLS_PRUNE << 30), 0);
-  // FIXED paths: table entries of rows past the end of the array are CLS_PRUNE, so no row bound
-  // is checked; destination element indices fit 32 bits (2 N * 45 < 2^32 for N < 23 M)
+  // table entries of rows past the end of the array are CLS_PRUNE, so no row bound is checked;
+  // destination element indices fit 32 bits (2 N * 45 < 2^32 for N < 23 M)
   constexpr bool plain = SET != 0 || A == 1 || A == 2;  // the new row is a copy (parameters) or zero (moments)
   auto emit_fixed = [&](int r, int col, int2 info, float val) {
     if constexpr (plain) {  // two predicated stores, no branches
@@ -353,25 +346,26 @@ __device__ __forceinline__ void rows_job(int row0, int rows_here, const int2 *__
       emit(r, col, info, val);
     }
   };
-  if constexpr (FIXED != 0 && w == 45) {
+  if constexpr (w == 45) {
     // Two rows = 90 elements = three rounds of 32 lanes (94 % of the lanes busy): which of the two
-    // rows and which column a lane handles in each round does not depend on the pair, so the
-    // division by 45 of the generic loop disappears; FIXED pairs (3 FIXED loads) in flight per lane.
+    // rows and which column a lane handles in each round does not depend on the pair, so no
+    // element index is divided by 45; DG_PAIRS pairs (3 DG_PAIRS loads) in flight per lane.
+    const int2 pruned = make_int2((int)((unsigned)CLS_PRUNE << 30), 0);
     const int rsel[3] = {0, lane >= 13, 1};
     const int col[3] = {lane, lane < 13 ? 32 + lane : lane - 13, 19 + lane};
 #pragma unroll 1
-    for (int p0 = 0; p0 < 16; p0 += FIXED) {
-      float v[FIXED][3];
-      int2 info[FIXED][3];
+    for (int p0 = 0; p0 < 16; p0 += DG_PAIRS) {
+      float v[DG_PAIRS][3];
+      int2 info[DG_PAIRS][3];
 #pragma unroll
-      for (int q = 0; q < FIXED; q++)
+      for (int q = 0; q < DG_PAIRS; q++)
 #pragma unroll
         for (int rd = 0; rd < 3; rd++) {
           info[q][rd] = tab[2 * (p0 + q) + rsel[rd]];
           if (rd == 2 && lane >= 26) info[q][rd] = pruned;  // 90 elements: the third round has 26
         }
 #pragma unroll
-      for (int q = 0; q < FIXED; q++)
+      for (int q = 0; q < DG_PAIRS; q++)
 #pragma unroll
         for (int rd = 0; rd < 3; rd++) {  // all loads are issued before any is consumed
           v[q][rd] = 0.f;
@@ -379,11 +373,11 @@ __device__ __forceinline__ void rows_job(int row0, int rows_here, const int2 *__
             v[q][rd] = __ldg(gsrc + (2 * (p0 + q) + rsel[rd]) * w + col[rd]);
         }
 #pragma unroll
-      for (int q = 0; q < FIXED; q++)
+      for (int q = 0; q < DG_PAIRS; q++)
 #pragma unroll
         for (int rd = 0; rd < 3; rd++) emit_fixed(2 * (p0 + q) + rsel[rd], col[rd], info[q][rd], v[q][rd]);
     }
-  } else if constexpr (FIXED != 0) {
+  } else {
     // w = 1, 3, 4: the whole group is w rounds of 32 lanes, row and column of a lane's element in
     // round u are the same for every group (hoisted out of the group loop by the compiler)
     float v[w];
@@ -400,31 +394,10 @@ __device__ __forceinline__ void rows_job(int row0, int rows_here, const int2 *__
       const int e = 32 * u + lane, r = e / w;
       emit_fixed(r, e - r * w, info[u], v[u]);
     }
-  } else {
-    constexpr int U = w >= 16 ? 8 : (w >= 3 ? 3 : 1);  // loads in flight per lane (w = 3: 96 elements = 3 rounds)
-    const int nelem = rows_here * w;
-#pragma unroll 1
-    for (int e0 = 0; e0 < nelem; e0 += 32 * U) {
-      float v[U];
-      int2 info[U];
-      int r[U];
-#pragma unroll
-      for (int u = 0; u < U; u++) {  // all loads are issued before any is consumed
-        const int e = e0 + 32 * u + lane;
-        info[u] = pruned;
-        r[u] = e / w;
-        if (e < nelem) {
-          info[u] = tab[r[u]];
-          if (((unsigned)info[u].x >> 30) != CLS_PRUNE) v[u] = __ldg(gsrc + e);
-        }
-      }
-#pragma unroll
-      for (int u = 0; u < U; u++) emit(r[u], e0 + 32 * u + lane - r[u] * w, info[u], v[u]);
-    }
   }
 }
 
-template <int A, int SET, int FIXED>
+template <int A, int SET>
 __device__ __noinline__ void rows_loop(int N, const uint8_t *__restrict__ cls, const Slot3 *__restrict__ slots, int K,
                                        int C, const Sets &S, const float *__restrict__ z, int2 *tab) {
   const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
@@ -440,12 +413,11 @@ __device__ __noinline__ void rows_loop(int N, const uint8_t *__restrict__ cls, c
     // (class | survivor slot, new-row slot); slots < N < 2^30
     tab[lane] = make_int2((int)((unsigned)c << 30) | sl.k, c == CLS_SPLIT ? K + C + sl.s : K + sl.c);
     __syncwarp();
-    rows_job<A, SET, FIXED>(row0, min(32, N - row0), tab, K, C, S, z, lane);
+    rows_job<A, SET>(row0, tab, K, C, S, z, lane);
     __syncwarp();  // the table is rewritten for the next group
   }
 }
 
-template <int FIXED>
 __global__ void __launch_bounds__(32 * DG_WARPS) k_density_apply_rows(int N, const uint8_t *__restrict__ cls,
                                                                        const Slot3 *__restrict__ slots, int K, int C,
                                                                        const __grid_constant__ Sets S,
@@ -453,7 +425,7 @@ __global__ void __launch_bounds__(32 * DG_WARPS) k_density_apply_rows(int N, con
   __shared__ int2 tabs[DG_WARPS][32];
   int2 *tab = tabs[threadIdx.x >> 5];
 #define GSB_JOB(y, a, s) \
-  case y: rows_loop<a, s, FIXED>(N, cls, slots, K, C, S, z, tab); break;
+  case y: rows_loop<a, s>(N, cls, slots, K, C, S, z, tab); break;
   switch (blockIdx.y) {
     GSB_JOB(0, 2, 0) GSB_JOB(1, 2, 1) GSB_JOB(2, 2, 2) GSB_JOB(3, 0, 0) GSB_JOB(4, 0, 1) GSB_JOB(5, 0, 2)
     GSB_JOB(6, 1, 0) GSB_JOB(7, 1, 1) GSB_JOB(8, 1, 2) GSB_JOB(9, 3, 0) GSB_JOB(10, 3, 1) GSB_JOB(11, 3, 2)
@@ -618,33 +590,20 @@ int launch_density_apply(int64_t N, const uint8_t *cls, const int32_t *slots, in
     S.dv[a] = dst_v ? dst_v[a] : nullptr;
   }
   ProfScope ps(K_DENSITY_APPLY, st);
-  static const int variant = [] {  // 3 (default) / 2 / 1 = row groups (see the launch below), 0 = one element per thread
-    const char *e = getenv("GSB_DENSITY_VARIANT");
-    return e != nullptr ? atoi(e) : GSB_DENSITY_DEFAULT_VARIANT;
-  }();
-  if (variant >= 1 && N < 23000000) {
+  if (N < 23000000) {
     int dev = 0, sms = 148;
     GSB_CUDA_TRY(cudaGetDevice(&dev));
     GSB_CUDA_TRY(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
     const int64_t blocks = (N + 32 * DG_WARPS - 1) / (32 * DG_WARPS);
     const int grid_x = (int)(blocks < (int64_t)sms * 8 ? blocks : (int64_t)sms * 8);
     const dim3 grid(grid_x, 18);
-    const Slot3 *sl = reinterpret_cast<const Slot3 *>(slots);
-    if (variant == 3)  // fixed lane -> (row, column) maps, 12 loads in flight per lane for the wide arrays
-      k_density_apply_rows<4><<<grid, 32 * DG_WARPS, 0, st>>>((int)N, cls, sl, (int)K, (int)C, S, z);
-    else if (variant == 2)  // the same with 6 loads in flight
-      k_density_apply_rows<2><<<grid, 32 * DG_WARPS, 0, st>>>((int)N, cls, sl, (int)K, (int)C, S, z);
-    else  // generic loop (one division per element)
-      k_density_apply_rows<0><<<grid, 32 * DG_WARPS, 0, st>>>((int)N, cls, sl, (int)K, (int)C, S, z);
+    k_density_apply_rows<<<grid, 32 * DG_WARPS, 0, st>>>((int)N, cls, reinterpret_cast<const Slot3 *>(slots), (int)K,
+                                                         (int)C, S, z);
     GSB_CUDA_TRY(cudaGetLastError());
     return 0;
   }
   dim3 grid(stream_grid((N * 45 + 3) / 4, 256), 18);
-  if (N < 23000000)
-    k_density_apply<int32_t><<<grid, 256, 0, st>>>((int32_t)N, cls, reinterpret_cast<const Slot3 *>(slots), (int32_t)K,
-                                                   (int32_t)C, S, z);
-  else
-    k_density_apply<int64_t><<<grid, 256, 0, st>>>(N, cls, reinterpret_cast<const Slot3 *>(slots), K, C, S, z);
+  k_density_apply<<<grid, 256, 0, st>>>(N, cls, reinterpret_cast<const Slot3 *>(slots), K, C, S, z);
   GSB_CUDA_TRY(cudaGetLastError());
   return 0;
 }

@@ -151,26 +151,22 @@ int launch_sort_and_pack(int H, int W, int N, int64_t P, uint32_t depth_key_max,
 int launch_pack_only(int64_t P, const int32_t *gsid_per_patch, const float *us, const float *cinv2ds,
                      const float *alphas, const float *colors, Rec *recs, cudaStream_t st);
 
-// ---- rasterizer (raster_fwd2.cu / raster_bwd2.cu + raster_bwd.cu).  recs: one 48-byte record per
-// Gaussian; gsid: the sorted patch list -- the kernels gather records into their stage buffers.
-int launch_draw_bwd2_kernel(int H, int W, const int32_t *ranges, const Rec *recs, const int32_t *gsid,
-                            const int32_t *contrib, const float *final_tau, const float *dloss_dgammas,
-                            float *moments, int *tile_counter, cudaStream_t st);
+// ---- rasterizer (raster_fwd3.cu, raster_bwd4.cu + raster_bwd.cu).  recs: one 48-byte record per
+// Gaussian; gsid: the sorted patch list -- every warp gathers the records of its tile's list itself.
+// work_counter: the work area of k_tile_list (below), which both rasterizers pull their items from.
 int launch_draw_bwd4_kernel(int H, int W, const int32_t *ranges, const Rec *recs, const int32_t *gsid,
                             const int32_t *contrib, const float *final_tau, const float *dloss_dgammas,
                             float *moments, int *work_counter, cudaStream_t st);
-int launch_draw(int H, int W, const int32_t *ranges, const Rec *recs, const int32_t *gsid, float *image,
-                int32_t *contrib, float *final_tau, int *tile_counter, int *work_counter, cudaStream_t st);
 // work = [item counter, #entries, entries ...] (2 + 4 * tiles ints, see k_tile_list); with outputs given the
 // empty tiles are zero-filled here
 int launch_tile_list(int H, int W, const int32_t *ranges, float *image, int32_t *contrib, float *final_tau,
                      int *work, cudaStream_t st);
-int launch_draw3(int H, int W, const int32_t *ranges, const Rec *recs, const int32_t *gsid, float *image,
-                 int32_t *contrib, float *final_tau, int *work_counter, cudaStream_t st);
+int launch_draw(int H, int W, const int32_t *ranges, const Rec *recs, const int32_t *gsid, float *image,
+                int32_t *contrib, float *final_tau, int *work_counter, cudaStream_t st);
 int launch_draw_backward(int H, int W, int N, const int32_t *ranges, const Rec *recs, const int32_t *gsid,
                          const int32_t *contrib,
                          const float *final_tau, const float *dloss_dgammas, const float *cinv2ds,
-                         float *moments, int *tile_counter, int *work_counter, float *dloss_dus,
+                         float *moments, int *work_counter, float *dloss_dus,
                          float *dloss_dcinv2ds, float *dloss_dalphas, float *dloss_dcolors, bool finalize,
                          cudaStream_t st);
 

@@ -9,14 +9,9 @@
 //                and the final loss scalar.
 // Algorithmic bytes: 24 (read img, gt) + 36 (write maps) + 36 + 24 (read) + 12 (write grad)
 // = 132 B per pixel (x3 channels already counted) -> HBM roofline.
-#include <stdlib.h>
-
 #include "common.cuh"
 #include "kernels.h"
 
-#ifndef GSB_LOSS_DEFAULT_VARIANT
-#define GSB_LOSS_DEFAULT_VARIANT 1
-#endif
 #ifndef GSB_LOSS_FWD_MINB  // resident CTAs (of 4 warps) the row kernels are compiled for
 #define GSB_LOSS_FWD_MINB 4
 #endif
@@ -209,9 +204,10 @@ __global__ void __launch_bounds__(256) k_ssim_bwd(int W, int H, const float *__r
 }
 
 // ---------------------------------------------------------------------------------------
-// Row-streaming variant (default).  The tiled kernels above spend 70 % of their instructions on
-// staging (index arithmetic, shared-memory traffic for both passes); here one lane owns one
-// image COLUMN and walks down a strip of rows:
+// Row streaming: k_ssim_fwd_rows / k_ssim_bwd_rows, the path for every image below 2^31 / 9
+// pixels (they use 32-bit element offsets; larger images take the tiled kernels above).  The
+// tiled kernels spend 70 % of their instructions on staging (index arithmetic, shared-memory
+// traffic for both passes); here one lane owns one image COLUMN and walks down a strip of rows:
 //   * a row of img and gt goes through a 48-column per-warp shared-memory line (the warp's 32
 //     columns + 8 either side, so that with W % 4 == 0 the line is 12 aligned float4 per image:
 //     ONE 16-byte load per lane and row); 22 LDS feed the 11 horizontal taps;
@@ -311,7 +307,7 @@ __global__ void __launch_bounds__(32 * SWARPS, GSB_LOSS_FWD_MINB) k_ssim_fwd_row
   const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
   const int x0 = (blockIdx.x * SWARPS + wid) * 32, x = x0 + lane;
   const int yb = blockIdx.y * SH, ye = min(yb + SH, H), c = blockIdx.z;
-  const int HW = H * W;  // (the host keeps H * W < 2^31 / 9 for this variant)
+  const int HW = H * W;  // (the host takes this kernel only for H * W < 2^31 / 9)
   float *__restrict__ mp0 = maps + (size_t)c * HW, *__restrict__ mp1 = mp0 + (size_t)3 * HW,
                       *__restrict__ mp2 = mp0 + (size_t)6 * HW;
   const bool xin = x < W;
@@ -469,13 +465,8 @@ __global__ void __launch_bounds__(32 * SWARPS, GSB_LOSS_BWD_MINB) k_ssim_bwd_row
 }
 
 // rows per strip: about one resident wave of warps (a strip pays 10 halo rows, so the longer the
-// better, but every SM needs its share); GSB_LOSS_STRIP overrides (A/B)
+// better, but every SM needs its share)
 static int strip_rows(int H, int W) {
-  static const int forced = [] {
-    const char *e = getenv("GSB_LOSS_STRIP");
-    return e != nullptr ? atoi(e) : 0;
-  }();
-  if (forced > 0) return forced;
   int dev = 0, sms = 148;
   if (cudaGetDevice(&dev) == cudaSuccess) cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
   const int xblocks = (W + 32 * SWARPS - 1) / (32 * SWARPS);
@@ -505,11 +496,8 @@ int launch_gau_loss(int H, int W, const float *img, const float *gt, float lambd
   double *acc = static_cast<double *>(ws);
   float *maps = reinterpret_cast<float *>(static_cast<char *>(ws) + 256);
   GSB_CUDA_TRY(cudaMemsetAsync(acc, 0, 2 * sizeof(double), st));
-  static const int variant = [] {  // 1 = row streaming (default), 0 = the tiled kernels (A/B)
-    const char *e = getenv("GSB_LOSS_VARIANT");
-    return e != nullptr ? atoi(e) : GSB_LOSS_DEFAULT_VARIANT;
-  }();
-  if (variant == 1 && (long long)H * W < (1ll << 31) / 9) {  // (int element offsets inside the kernels)
+  // the row kernels address the maps with 32-bit offsets; larger images take the tiled kernels
+  if ((long long)H * W < (1ll << 31) / 9) {
     const int SH = strip_rows(H, W);
     const dim3 grid((W + 32 * SWARPS - 1) / (32 * SWARPS), (H + SH - 1) / SH, 3);
     // 16-byte row loads need every row (and plane) of all five arrays 16-byte aligned

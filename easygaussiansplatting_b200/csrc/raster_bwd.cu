@@ -1,25 +1,14 @@
 // Backward tile rasterizer ("drawB").  Replaces reference kernel.cu:809-950.
 //
-// (The kernel itself is k_draw_bwd2 in raster_bwd2.cu; this file holds the algorithm notes, the
-// moment finalisation and the launcher.)
-// Same tiling and record pipeline as the forward (raster_fwd2.cu), walked back to front starting at the last
-// batch any pixel of the tile needs (max contrib).  Each pixel replays its saved
-// (final_tau, contrib) state: tau <- tau / (1 - alpha'), dL/dalpha' = tau (c - gamma_next) . dL/dgamma,
-// with gamma_next kept as the scalar s = dL/dgamma . gamma_next (s <- alpha' (dL/dgamma . c) + (1 - alpha') s).
-//
-// Geometry gradients are linear in per-pixel moments, so a pixel only produces nine numbers
+// This file holds the moment finalisation and the launcher; the kernel and its algorithm notes
+// are k_draw_bwd4 in raster_bwd4.cu.  Each pixel replays its saved (final_tau, contrib) state back
+// to front: tau <- tau / (1 - alpha'), dL/dalpha' = tau (c - gamma_next) . dL/dgamma, with
+// gamma_next kept as the scalar s = dL/dgamma . gamma_next (s <- alpha' (dL/dgamma . c) + (1 - alpha') s).
+// Geometry gradients are linear in per-pixel moments, so the kernel accumulates per Gaussian one
+// contiguous 9-float moment row
 //   w dx, w dy, w dx^2, w dx dy, w dy^2   (w = dL/dalpha' * alpha'),  dL/dalpha' * g,  alpha' tau dL/dgamma_rgb
-// which are summed over the 32 pixels of the warp with a SPLIT butterfly: at every level each
-// lane keeps half of the values and trades the other half, so the 9 sums cost 12 shuffles
-// (5+3+2+1+1) instead of 45, and end up in 9 different lanes.  Those 9 lanes then issue ONE
-// predicated red.global.add into the Gaussian's contiguous 9-float moment row (36 B, two
-// sectors) -- the reference issues 9 atomics per (pixel, record) into four arrays.
-// finalize_splat_grads() turns moment rows into the four gradient tensors:
+// and finalize_splat_grads() turns the rows into the four gradient tensors:
 //   dL/du = -(A Sx + B Sy, B Sx + C Sy),  dL/dconic = (-Sxx/2, -Sxy, -Syy/2).
-// Records that cannot touch the warp's rectangle are culled by the same ballot test as the
-// forward; records where no pixel is active are skipped before any reduction.
-#include <stdlib.h>
-
 #include "common.cuh"
 #include "kernels.h"
 #include "tile_io.cuh"
@@ -71,22 +60,15 @@ __global__ void __launch_bounds__(PG) k_finalize_grads(int N, const float *__res
 int launch_draw_backward(int H, int W, int N, const int32_t *ranges, const Rec *recs, const int32_t *gsid,
                          const int32_t *contrib,
                          const float *final_tau, const float *dloss_dgammas, const float *cinv2ds,
-                         float *moments, int *tile_counter, int *work_counter, float *dloss_dus,
+                         float *moments, int *work_counter, float *dloss_dus,
                          float *dloss_dcinv2ds, float *dloss_dalphas, float *dloss_dcolors, bool finalize,
                          cudaStream_t st) {
   const int gx = (W + TILE - 1) / TILE, gy = (H + TILE - 1) / TILE;
   if (gx <= 0 || gy <= 0 || N <= 0) return 0;
   GSB_CUDA_TRY(cudaMemsetAsync(moments, 0, sizeof(float) * MOM * (size_t)N, st));
   if (recs != nullptr) {
-    // GSB_BWD_VARIANT=2 selects the older warp-reduction kernel (raster_bwd2.cu) for A/B runs
-    static const int variant = [] {
-      const char *e = getenv("GSB_BWD_VARIANT");
-      return e != nullptr ? atoi(e) : 4;
-    }();
-    int rc = variant == 2   ? launch_draw_bwd2_kernel(H, W, ranges, recs, gsid, contrib, final_tau, dloss_dgammas,
-                                                      moments, tile_counter, st)
-                            : launch_draw_bwd4_kernel(H, W, ranges, recs, gsid, contrib, final_tau, dloss_dgammas,
-                                                      moments, work_counter, st);
+    int rc = launch_draw_bwd4_kernel(H, W, ranges, recs, gsid, contrib, final_tau, dloss_dgammas, moments,
+                                     work_counter, st);
     if (rc) return rc;
   }
   GSB_CUDA_TRY(cudaGetLastError());

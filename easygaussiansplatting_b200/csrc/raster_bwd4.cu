@@ -62,7 +62,7 @@ __device__ __forceinline__ float2 p2s(float a) { return make_float2(a, a); }
 __device__ __forceinline__ float2 lo(const float4 &v) { return make_float2(v.x, v.y); }
 __device__ __forceinline__ float2 hi(const float4 &v) { return make_float2(v.z, v.w); }
 
-// Phase B (identical to variant 3): moment sums of up to 8 records over the warp's 8x8 block.
+// Phase B: moment sums of up to 8 records over the warp's 8x8 block.
 //   lane = slot * 4 + part; part covers x in [4 (part & 1), +4) of rows (part >> 1) + {0, 2, 4, 6}.
 //   inf = record word q0 = (u_x, u_y, gaussian id, alpha) of the lane's slot.  It travels in registers:
 //   the kernel is bound by shared-memory wavefronts (ncu: LSU data pipe 89 %), and a 16-byte

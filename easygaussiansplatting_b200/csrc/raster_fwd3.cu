@@ -9,7 +9,8 @@
 // surviving records go into a small shared-memory list that the compositing loop walks two at a
 // time (two independent alpha' chains in flight per warp).  A lane owns two horizontally adjacent
 // pixels; the quadratic form, the alpha multiply and the compositing update are packed f32x2.
-// Per-pixel arithmetic is the instruction sequence of variant 2 (raster_fwd2.cu): identical images.
+// f3_alpha is the operation sequence of the backward's b4_eval (raster_bwd4.cu), so forward and
+// backward compute bit-identical alpha' and take the same skip decisions.
 // Replaces reference kernel.cu:152-271 (draw).
 #include "common.cuh"
 #include "kernels.h"
@@ -308,7 +309,7 @@ __global__ void __launch_bounds__(128, FWD3_MINBLOCKS) k_draw3(int W, int H, int
   }
 }
 
-int launch_draw3(int H, int W, const int32_t *ranges, const Rec *recs, const int32_t *gsid, float *image,
+int launch_draw(int H, int W, const int32_t *ranges, const Rec *recs, const int32_t *gsid, float *image,
                  int32_t *contrib, float *final_tau, int *work_counter, cudaStream_t st) {
   const int gx = (W + TILE - 1) / TILE, gy = (H + TILE - 1) / TILE;
   if (gx <= 0 || gy <= 0) return 0;

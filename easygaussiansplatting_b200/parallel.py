@@ -232,9 +232,6 @@ class GradExchange:
             self._own = None
 
 
-_EARLY_GATHER = __import__("os").environ.get("GSB_EARLY_GATHER", "1") != "0"  # A/B switch (bench)
-
-
 class MultiViewStep:
     """One data-parallel training step over the views of all ranks with the FACTORISED gradient sum.
 
@@ -281,7 +278,7 @@ class MultiViewStep:
                              ranges, gsid, dloss_dimage, moments_only=True)
         self._colors.append(moments[:, 6:9])          # dL/dcolor of this view
         self._twcs.append(cam.twc.reshape(1, 3))
-        if last and self.world > 1 and _EARLY_GATHER:
+        if last and self.world > 1:
             self._early = _start_gathers(torch.stack(self._colors), torch.cat(self._twcs).contiguous(), self.group)
         gpw, _, gs, gq, dus, dal = ops.preprocessB(
             self.pws, self.rots, self.scales, self.shs, cam.Rcw, cam.tcw, cam.twc, cam.fx, cam.fy, cam.cx, cam.cy,

@@ -58,16 +58,26 @@ def test_no_library_kernels_and_host_only_entry_points():
     assert lib.gsb_splat_workspace_bytes(1000, 64, 64, 10) <= lib.gsb_splat_workspace_bytes(1000, 64, 64, 100000)
 
 
-def test_library_is_sm100a_with_async_record_gather():
-    """built for sm_100a; the rasterizers stage records with 16-byte async copies tracked by an
-    mbarrier (SASS LDGSTS + LDGSTSBAR arrive-on + SYNCS try-wait) and use packed fp32 math"""
+def test_rasterizers_are_sm100a_with_cp_async_record_gather():
+    """built for sm_100a; each rasterizer kernel gathers its records with 16-byte cp.async copies
+    waited on per group (SASS LDGSTS + LDGDEPBAR) and uses packed fp32 math; the library reads no
+    user-set kernel switch from the environment"""
     from easygaussiansplatting_b200 import _lib, build
     build.build()
     r = subprocess.run(["cuobjdump", "-sass", _lib.LIB_PATH], capture_output=True, text=True)
     assert "code for sm_100a" in r.stdout
-    assert "LDGSTS.E.BYPASS.128" in r.stdout and "LDGSTSBAR" in r.stdout, "async record gather missing"
-    assert "SYNCS.PHASECHK" in r.stdout, "mbarrier wait missing"
-    assert "FFMA2" in r.stdout and "MUFU.EX2" in r.stdout
+    sass = {}
+    for part in re.split(r"^\s+Function : ", r.stdout, flags=re.M)[1:]:
+        name, body = part.split("\n", 1)
+        sass[name.strip()] = body
+    for kernel in ("k_draw3", "k_draw_bwd4"):
+        found = [n for n in sass if re.search(r"\d%sE" % kernel, n)]
+        assert len(found) == 1, (kernel, found)
+        body = sass[found[0]]
+        for ins in ("LDGSTS.E.BYPASS.128", "LDGDEPBAR", "FFMA2", "MUFU.EX2"):
+            assert ins in body, "%s: %s missing" % (kernel, ins)
+    strings = re.findall(rb"[\x20-\x7e]{4,}", open(_lib.LIB_PATH, "rb").read())
+    assert sorted({s.decode() for s in strings if s.startswith(b"GSB_")}) == ["GSB_EXCHANGE_TIMEOUT_S"]
 
 
 def test_ops_refuse_cpu_tensors():

@@ -79,8 +79,7 @@ class RowFetch:
                 if st:
                     self.line[m][buf][d:d + len(v)] = v
 
-def strip_rows(H, W, sms=148, forced=0):
-    if forced: return forced
+def strip_rows(H, W, sms=148):
     xblocks = (W + 32 * SWARPS - 1) // (32 * SWARPS)
     strips = max(1, (sms * 4) // (3 * xblocks))
     sh = (H + strips - 1) // strips
@@ -239,7 +238,7 @@ def random_state(N, seed, sense=5.0):
     cnt = rng.integers(0, 6, N).astype(np.int32); acc[cnt == 0] = 0
     return P, M, acc, cnt
 
-def rows_job(w, src, dst, row0, rows_here, tab, K, C, newval):
+def rows_job(w, src, dst, row0, tab, K, C, newval):
     gsrc = src[row0 * w:]
     def emit(r, col, info, val):
         cl = (info[0] & 0xffffffff) >> 30
@@ -251,7 +250,7 @@ def rows_job(w, src, dst, row0, rows_here, tab, K, C, newval):
         assert np.isnan(dst[d]); dst[d] = newval(val, cl == SPLIT, row0 + r, info[1] - K - C, col)
     pruned = (PRUNE << 30, 0)
     # (table entries of rows past the end of the array are PRUNE: no row bound is checked)
-    if w == 45:  # FIXED = 4 row pairs, i.e. 12 loads, in flight per lane
+    if w == 45:  # DG_PAIRS = 4 row pairs, i.e. 12 loads, in flight per lane
         for p0 in range(0, 16, 4):
             for lane in range(32):
                 rsel = [0, 1 if lane >= 13 else 0, 1]
@@ -297,7 +296,7 @@ def test_density_row_group_schedule(N, seed):
                     c, sl = PRUNE, (0, 0, 0)
                     if row < N: c, sl = int(cls[row]), tuple(int(x) for x in slots[row])
                     tab.append(((c << 30) | sl[0], K + C + sl[2] if c == SPLIT else K + sl[1]))
-                rows_job(w, src, dst, row0, min(32, N - row0), tab, K, C, nv)
+                rows_job(w, src, dst, row0, tab, K, C, nv)
             assert not np.isnan(dst).any(), (name, setname)
             got = dst.reshape(-1, w)
             if setname == "m":
